@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the GP-PDE Gauss-Newton hot path (BASELINE.json metric: Gauss-Newton steps/sec).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--N_domain 40000]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--N_domain 40000] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input: Gram assembly -> Cholesky -> interior
 inverse -> GNsteps Gauss-Newton steps of the nonlinear elliptic problem (BASELINE configs[4]: N_domain collocation
@@ -21,6 +21,7 @@ N > 1 (torchrun): ONE problem sharded over the N GPUs (csrc/dist.cu), "scaling":
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import math
 import os
@@ -80,6 +81,7 @@ class ClockSampler:
         try:
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={q}", "--format=csv,noheader,nounits", "-i", str(self.index),
                                           "-lms", "200"], stdout=subprocess.PIPE, stderr=subprocess.DEVNULL, text=True)
+            atexit.register(self._end)      # also when a step raises before stop(): the sampler never outlives the benchmark
             threading.Thread(target=self._read, daemon=True).start()
         except Exception:
             self.proc = None
@@ -88,10 +90,21 @@ class ClockSampler:
         for line in self.proc.stdout:
             self.rows.append([c.strip() for c in line.split(",")])
 
+    def _end(self):
+        """Stop nvidia-smi and reap it, with SIGKILL when SIGTERM has not ended it within 5 s."""
+        if self.proc is None or self.proc.poll() is not None:
+            return
+        self.proc.terminate()
+        try:
+            self.proc.wait(timeout=5)
+        except subprocess.TimeoutExpired:
+            self.proc.kill()
+            self.proc.wait()
+
     def stop(self):
         if self.proc is None:
             return {"sm_mhz": None, "sm_max_mhz": None, "reasons": ["nvidia-smi unavailable"]}
-        self.proc.terminate()
+        self._end()
         sm, mx, reasons = [], [], set()
         names = ["hw_slowdown", "hw_thermal_slowdown", "sw_thermal_slowdown", "sw_power_cap"]
         for r in self.rows:
@@ -134,6 +147,13 @@ def hbm_peak():
     if os.path.exists(p):
         return float(json.load(open(p))["hbm_gbs"]), "of measured (MEASURED_PEAKS.json)"
     return HBM_PEAK_FALLBACK_GBS, "of fallback"
+
+
+def dump_outputs(out_dir, arrays):
+    """Each array as out_dir/<name>.npy in float64; at N_domain=40000 the four arrays come to 1.3 MB."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(v, dtype=np.float64))
 
 
 def cpu_port_solve(N_sample, gn_steps, nugget, solve="lu"):
@@ -216,7 +236,14 @@ def main():
     ap.add_argument("--skip_cpu_baseline", action="store_true")
     ap.add_argument("--NB", type=int, default=0)
     ap.add_argument("--Q", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last step returned (loss history, GN iterate, solution vector, "
+                         "collocation-point errors) as DIR/<name>.npy in float64")
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -338,6 +365,9 @@ def main():
     wall = time.perf_counter() - t0
     launches = eng.launch_count() - l0
     clocks = sampler.stop()
+    if a.dump_outputs and rank == 0:
+        # the inputs depend only on the arguments (seeded points and initial guess), so two builds can be compared array by array
+        dump_outputs(a.dump_outputs, {"loss_hist": prob.loss_hist, "sol": prob.sol, "sol_vec": prob.sol_vec, "pts_err": s.pts_err_all})
     red = maxred([dev_ms / 1e3, wall] + [phase[k] for k in ("assembly_ms", "potrf_ms", "inverse_ms", "gn_ms")])
     elapsed, e2e_elapsed = red[0], red[1]
     T_asm, T_potrf, T_inv, T_gn = [v / a.steps for v in red[2:]]

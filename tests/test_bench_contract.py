@@ -1,9 +1,12 @@
-"""bench.py contract checks that run without a GPU: the reference arm (CPU port on a bounded sample) prints one
-JSON line with the required keys; under torchrun only rank 0 prints."""
+"""bench.py contract checks.  Without a GPU: the reference arm (CPU port on a bounded sample) prints one JSON line with
+the required keys; under torchrun only rank 0 prints.  On the GPU: --dump-outputs writes what the timed path returned."""
 import json
 import os
 import subprocess
 import sys
+
+import numpy as np
+import pytest
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REQUIRED = ["impl", "metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling",
@@ -43,3 +46,22 @@ def test_reference_arm_under_torchrun_only_rank0_prints():
     assert len(lines) == 1
     _check(lines[0])
     assert json.loads(lines[0])["n_gpus"] == 2
+
+
+@pytest.mark.gpu
+def test_dump_outputs_are_the_last_timed_step(tmp_path):
+    """--dump-outputs writes the loss history, GN iterate, solution vector and collocation errors of the last timed step
+    in float64; they are the numbers the JSON line of the same run reports."""
+    out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "0", "--N_domain", "2000",
+                          "--nugget", "1e-8", "--skip_cpu_baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=600)
+    assert out.returncode == 0, out.stderr[-1500:]
+    lines = [l for l in out.stdout.splitlines() if l.startswith("{")]
+    assert len(lines) == 1
+    j = json.loads(lines[0])
+    assert j["steps"] == 2
+    d = {n: np.load(tmp_path / f"{n}.npy") for n in ("loss_hist", "sol", "sol_vec", "pts_err")}
+    assert all(v.dtype == np.float64 for v in d.values())
+    N, M = j["config"]["n"], j["config"]["M"]
+    assert d["loss_hist"].shape == (5,) and d["sol"].shape == (N,) and d["sol_vec"].shape == (M,) and d["pts_err"].shape == (N,)
+    assert d["loss_hist"][-1] == j["result"]["final_loss"] and d["pts_err"].max() == j["result"]["pts_max_err"]
