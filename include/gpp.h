@@ -121,6 +121,12 @@ int gpp_dist_info(gpp_handle* h, int* rank, int* world, int* P, int* Q);
  * that a step must solve / update is handled by exactly one rank, its owner.  phase 0 Cholesky, 1 U = L^-T, 2 Theta^-1
  * sub-blocks (n = N_domain, nb_extra = boundary rows).  0 = consistent. */
 int gpp_dist_plan_check(int n, int NB, int P, int Q, int phase, int nb_extra);
+/* host-only self-check of the Theta^-1 sub-block plans of a PDE's sharded Hessian (pde GPP_PDE_ELLIPTIC, _BURGERS or
+ * _EIKONAL; N = N_domain, nb_extra = boundary rows): every lower block of the nz N x nz N Hessian has exactly one owner, and
+ * every element of it receives each term of its unknown-block pair exactly once, from the right operand rows and K range.
+ * Blocks that straddle the boundary between two unknown fields (N % NB != 0) are split into one-field segments.
+ * 0 = consistent, -1 = bad argument or a PDE that does not shard.  Phase 2 of gpp_dist_plan_check is the elliptic case. */
+int gpp_dist_hess_plan_check(int N, int NB, int P, int Q, int pde, int nb_extra);
 /* how finished panels travel: 1 = peer-to-peer (the solve kernels store every finished tile straight into the peers'
  * replicated buffers over NVLink through CUDA IPC mappings and announce it by flags), 0 = NCCL all-gather / broadcast
  * (GPP_DIST_P2P=0, or CUDA IPC unavailable) */
@@ -134,11 +140,14 @@ int gpp_dist_add_diag(gpp_handle* h, const double* add);
 /* distributed X.Gram_Cholesky of slot 0 (right-looking, look-ahead, one panel gather per block column).  Afterwards every
  * rank holds the whole factor: gpp_gn_loss, gpp_solve_vec, gpp_predict, gpp_gram_download(h, 0, 1, .) work on any rank. */
 int gpp_dist_potrf(gpp_handle* h, int* info);
-/* distributed counterpart of gpp_inverse (elliptic layout): U = L^{-T} sharded then replicated, and the sub-blocks of the
- * interior block of Theta^{-1} that this rank's Hessian blocks need */
+/* distributed counterpart of gpp_inverse (elliptic, Burgers and Eikonal layouts; the Darcy layouts are refused): U = L^{-T}
+ * sharded then replicated, and the sub-blocks of the interior block of Theta^{-1} that this rank's Hessian blocks need for
+ * the PDE of the layout in slot 0 */
 int gpp_dist_inverse(gpp_handle* h);
 /* gpp_gn_step with the Hessian assembled block-wise by the owners and factorised by the distributed Cholesky; z and the
- * returned loss are identical on every rank (PDE id GPP_PDE_ELLIPTIC only) */
+ * returned loss are identical on every rank.  PDE ids GPP_PDE_ELLIPTIC, GPP_PDE_BURGERS and GPP_PDE_EIKONAL (the relaxed
+ * method and Darcy are refused); the PDE of gpp_gn_setup must be the one of the layout gpp_dist_inverse planned for,
+ * otherwise -5 */
 int gpp_dist_gn_step(gpp_handle* h, double step_size, double* loss);
 
 #ifdef __cplusplus

@@ -63,9 +63,9 @@ class _GPProblem(object):
         the inverse and the GN Hessian are then owner-computes over a P x Q block-cyclic grid with NCCL panel gathers
         (csrc/dist.cu); all results (loss history, solution, predictions) are identical on every rank.
         ``virtual_ranks=n`` instead emulates n ranks on this one GPU (tests)."""
-        if self._eqn != 'Nonlinear_elliptic':
-            raise NotImplementedError("the sharded path covers Nonlinear_elliptic2d (BASELINE configs[4]); "
-                                      "the small configurations are latency-bound and run as replicas")
+        if self._eqn not in ('Nonlinear_elliptic', 'Burgers'):
+            raise NotImplementedError("the sharded path covers Nonlinear_elliptic2d and Burgers (not Eikonal, "
+                                      "Darcy_flow2d or the relaxed method)")
         eng = self._engine()
         if virtual_ranks is not None:
             eng.dist_init_virtual(virtual_ranks)

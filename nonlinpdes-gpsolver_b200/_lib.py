@@ -63,6 +63,7 @@ def _sig(lib):
         "gpp_dist_info": [H, _ip, _ip, _ip, _ip],
         "gpp_dist_exchange_mode": [H],
         "gpp_dist_plan_check": [C.c_int] * 6,
+        "gpp_dist_hess_plan_check": [C.c_int] * 6,
         "gpp_dist_finalize": [H],
         "gpp_dist_gram_assemble": [H, C.c_int, C.c_int, _dp],
         "gpp_dist_get_diag": [H, _dp],
@@ -380,6 +381,11 @@ class Engine:
 def dist_plan_check(n, NB, P, Q=1, phase=0, nb_extra=0):
     """Host-only consistency check of the sharded task plans (works without a GPU); 0 = consistent."""
     return int(load().gpp_dist_plan_check(int(n), int(NB), int(P), int(Q), int(phase), int(nb_extra)))
+
+
+def dist_hess_plan_check(N, NB, P, Q=1, pde="Burgers", nb_extra=0):
+    """Host-only check of the Theta^-1 sub-block plans of a PDE's sharded Hessian (works without a GPU); 0 = consistent."""
+    return int(load().gpp_dist_hess_plan_check(int(N), int(NB), int(P), int(Q), PDE[pde], int(nb_extra)))
 
 
 def nccl_unique_id():

@@ -389,7 +389,7 @@ int gpp_gn_setup(gpp_handle* h, int pde, const double* params, const double* rhs
   GnState& g = h->gn;
   const int N = h->N, Nb = h->Nb;
   g.pde = pde;
-  g.nz = (pde == PDE_ELLIPTIC) ? 1 : (pde == PDE_DARCY ? 6 : (pde == PDE_ELLIPTIC_RELAXED ? 2 : 3));
+  g.nz = pde_nz(pde);
   g.n = g.nz * N;
   memset(g.params, 0, sizeof(g.params));
   g.m_int = 0;

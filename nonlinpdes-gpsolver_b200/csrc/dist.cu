@@ -48,8 +48,9 @@ inline bool mine(const Grid& g, int bi, int bc) { return bi % g.P == g.p && bc %
 struct Launch { size_t off = 0; int count = 0; };
 
 // Task lists of one phase for one (virtual) rank; built once per (size, NB, grid) and kept on the device.
+constexpr int kKeyLen = 9;
 struct Plan {
-  long key[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  long key[kKeyLen] = {0};
   bool valid = false;
   std::vector<GemmTask> host;
   GemmTask* dev = nullptr;
@@ -78,6 +79,7 @@ struct DistState {
   cudaStream_t sC = nullptr;     // communication stream of the U phase
   std::map<int, Plan> plans;     // key: phase * 4096 + virtual rank
   bool inverse_ready = false;
+  int inv_pde = -1;              // PDE whose Hessian the sub-block plan of the last gpp_dist_inverse serves
   // peer-to-peer path (GPP_DIST_P2P=1): the replicated buffers of all ranks are mapped into every process (CUDA IPC);
   // finished blocks are stored straight into the peers' copies over NVLink by the solve kernel and announced by flags.
   // Measured on 8 B200 (profiles/r02b_dist8_*.log): 3.79 s per N=40k solve against 2.98 s with the NCCL all-gather --
@@ -230,12 +232,12 @@ Plan& plan_slot(DistState* d, int phase, int vr) { return d->plans[phase * 4096 
 
 bool plan_matches(Plan& pl, const long* key) {
   if (!pl.valid) return false;
-  for (int k = 0; k < 8; ++k) if (pl.key[k] != key[k]) return false;
+  for (int k = 0; k < kKeyLen; ++k) if (pl.key[k] != key[k]) return false;
   return true;
 }
 
 void plan_reset(Plan& pl, const long* key) {
-  for (int k = 0; k < 8; ++k) pl.key[k] = key[k];
+  for (int k = 0; k < kKeyLen; ++k) pl.key[k] = key[k];
   pl.host.clear(); pl.la.clear(); pl.bulkA.clear(); pl.bulkB.clear(); pl.trsm.clear(); pl.rows.clear(); pl.hblocks.clear();
   pl.all = Launch{};
   pl.valid = false;
@@ -348,34 +350,74 @@ void build_uinv_plan(Plan& pl, const Grid& g, int n, int NB) {
   }
 }
 
-// sub-blocks of the interior inverse needed by the own Hessian blocks (elliptic layout: 2 operator blocks, H is N x N)
-void build_ablock_plan(Plan& pl, const Grid& g, int N, int M, const int* off, int nbh) {
-  const int nblk = nblocks_of(N, nbh);
+// PDEs whose Hessian the sharded GN step assembles, by the layout of their (single) Gram system; -1: not sharded
+int sharded_pde_of_layout(int layout) {
+  switch (layout) {
+    case LAY_ELLIPTIC: return PDE_ELLIPTIC;
+    case LAY_BURGERS: return PDE_BURGERS;
+    case LAY_EIKONAL: return PDE_EIKONAL;
+    default: return -1;
+  }
+}
+
+// Rows [b NB, b NB + NB) of the nz N x nz N Hessian cut where the unknown field changes: field q, first index i0 within
+// the field, first row r0 within the block, length len.  A block straddles a field boundary when N % NB != 0.
+struct Seg { int q, i0, r0, len; };
+std::vector<Seg> field_segments(int b, int NB, int n, int N) {
+  std::vector<Seg> v;
+  const int g0 = b * NB, g1 = std::min(g0 + NB, n);
+  for (int r = g0; r < g1;) {
+    const int q = r / N, e = std::min(g1, (q + 1) * N);
+    v.push_back(Seg{q, r - q * N, r - g0, e - r});
+    r = e;
+  }
+  return v;
+}
+
+// sub-blocks of the interior inverse needed by the own Hessian blocks: for every pair of field segments of an own block
+// and every term t = (p, p') of their pair (q, q'), A_pp'(i, j) = sum_k U[off[p] + i, k] U[off[p'] + j, k] lands in slot t
+// (of four) of the block's group in the compact store.  Every pair of elliptic, Burgers and Eikonal has at most four terms.
+// Elliptic (one field, four terms everywhere) gives exactly one task per (block, p, p').
+void build_ablock_plan(Plan& pl, const Grid& g, const TermTable& tt, int N, int M, const int* off, int nbh) {
+  const int n = tt.nz * N, nblk = nblocks_of(n, nbh);
   for (int bi = 0; bi < nblk; ++bi)
     for (int bc = 0; bc <= bi; ++bc)
       if (mine(g, bi, bc)) pl.hblocks.push_back(make_int4(bi, bc, (int)pl.hblocks.size(), 0));
   pl.all.off = 0;
   const int k1 = (int)round_up(M, 16);
-  for (const int4& hb : pl.hblocks)
-    for (int p = 0; p < 2; ++p)
-      for (int pp = 0; pp < 2; ++pp) {
-        const int a_row = off[p] + hb.x * nbh, b_row = off[pp] + hb.y * nbh;
-        const int k0 = (std::max(a_row, b_row) / 16) * 16;
-        pl.host.push_back(make_task(a_row, b_row, (hb.z * 4 + p * 2 + pp) * nbh, 0, rows_of(N, nbh, hb.x), rows_of(N, nbh, hb.y), k0, k1, 0, 0));
+  for (const int4& hb : pl.hblocks) {
+    const std::vector<Seg> rs = field_segments(hb.x, nbh, n, N), cs = field_segments(hb.y, nbh, n, N);
+    for (const Seg& a : rs)
+      for (const Seg& b : cs) {
+        const int pr = a.q * tt.nz + b.q;
+        for (int t = 0; t < tt.nterms[pr]; ++t) {
+          const int a_row = off[tt.tp[pr][t]] + a.i0, b_row = off[tt.tpp[pr][t]] + b.i0;
+          const int k0 = (std::max(a_row, b_row) / 16) * 16;      // U is upper triangular
+          pl.host.push_back(make_task(a_row, b_row, (hb.z * 4 + t) * nbh + a.r0, b.r0, a.len, b.len, k0, k1, 0, 0));
+        }
       }
+  }
   // longest K first: the hardware scheduler then balances the variable-length tiles
   std::stable_sort(pl.host.begin(), pl.host.end(), [](const GemmTask& a, const GemmTask& b) { return (a.k1 - a.k0) > (b.k1 - b.k0); });
   pl.all.count = (int)pl.host.size();
 }
 
-int ensure_plan(gpp_handle* h, DistState* d, int phase, int vr, const Grid& g, int n, int NB, int extraM, const int* off, Plan** out) {
+// phase 2: n = N_domain, extraM = M, off = the layout's row offsets, pde = the sharded PDE of that layout (else -1)
+int ensure_plan(gpp_handle* h, DistState* d, int phase, int vr, const Grid& g, int n, int NB, int extraM, const int* off, int pde,
+                Plan** out) {
   Plan& pl = plan_slot(d, phase, vr);
-  const long key[8] = {phase, n, NB, g.P, g.Q, g.p * 65536L + g.q, extraM, off ? off[1] : 0};
+  const long key[kKeyLen] = {phase, n, NB, g.P, g.Q, g.p * 65536L + g.q, extraM, off ? off[1] : 0, pde};
   if (!plan_matches(pl, key)) {
     plan_reset(pl, key);
-    if (phase == 0 || phase == 3) build_potrf_plan(pl, g, n, NB);
-    else if (phase == 1) build_uinv_plan(pl, g, n, NB);
-    else build_ablock_plan(pl, g, n, extraM, off, NB);
+    if (phase == 0 || phase == 3) {
+      build_potrf_plan(pl, g, n, NB);
+    } else if (phase == 1) {
+      build_uinv_plan(pl, g, n, NB);
+    } else {
+      TermTable tt;
+      if (make_term_table(pde, &tt) || tt.nslots != 1) { h->err = "sub-block plan: PDE not sharded"; return -1; }
+      build_ablock_plan(pl, g, tt, n, extraM, off, NB);
+    }
     int rc = plan_upload(h, pl);
     if (rc) return rc;
   }
@@ -598,7 +640,7 @@ int dist_potrf_matrix(gpp_handle* h, DistState* d, double* A, long ld, int n, co
   const std::vector<Grid> grids = grids_of(d);
   std::vector<Plan*> plans(grids.size());
   for (size_t v = 0; v < grids.size(); ++v) {
-    int rc = ensure_plan(h, d, phase, d->nv > 0 ? (int)v : 0, grids[v], n, NB, 0, nullptr, &plans[v]);
+    int rc = ensure_plan(h, d, phase, d->nv > 0 ? (int)v : 0, grids[v], n, NB, 0, nullptr, -1, &plans[v]);
     if (rc) return rc;
   }
   int rc = ensure_staging(h, d, n, NB);
@@ -759,7 +801,7 @@ int dist_uinv(gpp_handle* h, DistState* d, GramSlot& s) {
   const std::vector<Grid> grids = grids_of(d);
   std::vector<Plan*> plans(grids.size());
   for (size_t v = 0; v < grids.size(); ++v) {
-    int rc = ensure_plan(h, d, 1, d->nv > 0 ? (int)v : 0, grids[v], n, NB, 0, nullptr, &plans[v]);
+    int rc = ensure_plan(h, d, 1, d->nv > 0 ? (int)v : 0, grids[v], n, NB, 0, nullptr, -1, &plans[v]);
     if (rc) return rc;
   }
   int rc = ensure_staging(h, d, n, NB);
@@ -894,7 +936,7 @@ int dist_ablocks(gpp_handle* h, DistState* d, GramSlot& s) {
   size_t total_blocks = 0;
   std::vector<Plan*> plans(grids.size());
   for (size_t v = 0; v < grids.size(); ++v) {
-    int rc = ensure_plan(h, d, 2, d->nv > 0 ? (int)v : 0, grids[v], s.N, NB, s.M, s.off, &plans[v]);
+    int rc = ensure_plan(h, d, 2, d->nv > 0 ? (int)v : 0, grids[v], s.N, NB, s.M, s.off, d->inv_pde, &plans[v]);
     if (rc) return rc;
     total_blocks += plans[v]->hblocks.size();
   }
@@ -1042,36 +1084,91 @@ int gpp_dist_info(gpp_handle* h, int* rank, int* world, int* P, int* Q) {
   return GPP_OK;
 }
 
+// Host-only check of the Theta^{-1} sub-block plans of a PDE's sharded Hessian (no GPU, no handle): builds the plans of all
+// P * Q ranks for N = N_domain, block size NB and M = (operator blocks) N + nb_extra, and verifies for the nz N x nz N
+// Hessian that every lower block has exactly one owner and that every element of an own block receives each term of its
+// unknown-block pair exactly once, from the right operand rows and K range.  Returns 0, -1 on bad arguments or a PDE that
+// does not shard, or a positive code identifying the first violated property.
+int gpp_dist_hess_plan_check(int N, int NB, int P, int Q, int pde, int nb_extra) {
+  if (N <= 0 || NB <= 0 || NB % 64 || P < 1 || Q < 1 || P * Q > 64 || nb_extra < 0) return -1;
+  const int layout = pde == PDE_ELLIPTIC ? LAY_ELLIPTIC : pde == PDE_BURGERS ? LAY_BURGERS : pde == PDE_EIKONAL ? LAY_EIKONAL : -1;
+  TermTable tt;
+  if (layout < 0 || make_term_table(pde, &tt) || tt.nslots != 1) return -1;
+  const Layout lay = make_layout(layout);
+  int off[GPP_MAX_BLOCKS + 1] = {0};
+  for (int p = 0; p <= lay.nblk; ++p) off[p] = p * N;
+  const int M = lay.nblk * N + nb_extra, k1 = (int)round_up(M, 16);
+  const int n = tt.nz * N, nblk = nblocks_of(n, NB);
+  std::vector<Plan> plans(P * Q);
+  std::vector<Grid> grids;
+  for (int r = 0; r < P * Q; ++r) grids.push_back(Grid{P, Q, r / Q, r % Q});
+  for (int r = 0; r < P * Q; ++r) build_ablock_plan(plans[r], grids[r], tt, N, M, off, NB);
+  std::vector<int> cnt((size_t)nblk * nblk, 0);
+  std::vector<unsigned char> w((size_t)4 * NB * NB);
+  for (int r = 0; r < P * Q; ++r) {
+    const Plan& pl = plans[r];
+    std::vector<std::vector<const GemmTask*>> of_block(pl.hblocks.size());
+    size_t want_tasks = 0;
+    for (const int4& hb : pl.hblocks) {
+      if (owner_of(grids[r], hb.x, hb.y) != r || hb.y > hb.x) return 21;
+      cnt[(size_t)hb.x * nblk + hb.y]++;
+      for (const Seg& a : field_segments(hb.x, NB, n, N))
+        for (const Seg& b : field_segments(hb.y, NB, n, N)) want_tasks += tt.nterms[a.q * tt.nz + b.q];
+    }
+    if (pl.host.size() != want_tasks) return 20;        // elliptic: four tasks per Hessian block
+    for (const GemmTask& t : pl.host) {
+      const size_t e = (size_t)(t.c_row / (4 * NB));
+      if (t.c_row < 0 || e >= of_block.size()) return 23;
+      of_block[e].push_back(&t);
+    }
+    for (size_t e = 0; e < pl.hblocks.size(); ++e) {
+      const int4 hb = pl.hblocks[e];
+      const int rows = rows_of(n, NB, hb.x), cols = rows_of(n, NB, hb.y);
+      std::fill(w.begin(), w.end(), 0);
+      for (const GemmTask* t : of_block[e]) {
+        const int slot = (t->c_row / NB) % 4, r0 = t->c_row % NB, c0 = t->c_col;
+        if (t->m <= 0 || t->n <= 0 || c0 < 0 || r0 + t->m > rows || c0 + t->n > cols) return 23;
+        if (t->k0 != (std::max(t->a_row, t->b_row) / 16) * 16 || t->k1 != k1 || t->kb_off != 0 || t->tri != 0) return 24;
+        for (int x = 0; x < t->m; ++x) {
+          const int gr = hb.x * NB + r0 + x, q = gr / N, i = gr - q * N;
+          for (int y = 0; y < t->n; ++y) {
+            const int gc = hb.y * NB + c0 + y, qq = gc / N, j = gc - qq * N;
+            const int pr = q * tt.nz + qq;
+            if (slot >= tt.nterms[pr]) return 23;
+            if (t->a_row + x != off[tt.tp[pr][slot]] + i || t->b_row + y != off[tt.tpp[pr][slot]] + j) return 24;
+            w[((size_t)slot * NB + r0 + x) * NB + c0 + y]++;
+          }
+        }
+      }
+      for (int x = 0; x < rows; ++x)
+        for (int y = 0; y < cols; ++y) {
+          const int pr = ((hb.x * NB + x) / N) * tt.nz + (hb.y * NB + y) / N;
+          for (int slot = 0; slot < 4; ++slot)
+            if (w[((size_t)slot * NB + x) * NB + y] != (slot < tt.nterms[pr] ? 1 : 0)) return 25;
+        }
+    }
+  }
+  for (int bi = 0; bi < nblk; ++bi)
+    for (int bc = 0; bc <= bi; ++bc)
+      if (cnt[(size_t)bi * nblk + bc] != 1) return 22;
+  return 0;
+}
+
 // Host-only consistency check of the task plans (no GPU, no handle): builds the plans of all P * Q ranks for an n x n
 // matrix with block size NB and verifies, for every step, that each block that must be touched is touched by exactly one
 // rank (its owner) -- panel blocks solved once, trailing blocks updated once, Hessian blocks owned once.
-// phase: 0 = right-looking Cholesky, 1 = U = L^{-T}, 2 = Theta^{-1} sub-blocks (n = N_domain, M = 2 n + nb_extra).
-// Returns 0, or a positive code identifying the first violated property.
+// phase: 0 = right-looking Cholesky, 1 = U = L^{-T}, 2 = Theta^{-1} sub-blocks of the elliptic Hessian (n = N_domain,
+// M = 2 n + nb_extra; gpp_dist_hess_plan_check).  Returns 0, or a positive code identifying the first violated property.
 int gpp_dist_plan_check(int n, int NB, int P, int Q, int phase, int nb_extra) {
   if (n <= 0 || NB <= 0 || NB % 64 || P < 1 || Q < 1 || P * Q > 64 || phase < 0 || phase > 2) return -1;
+  if (phase == 2) return gpp_dist_hess_plan_check(n, NB, P, Q, PDE_ELLIPTIC, nb_extra);
   const int nblk = nblocks_of(n, NB);
   std::vector<Plan> plans(P * Q);
   std::vector<Grid> grids;
   for (int r = 0; r < P * Q; ++r) grids.push_back(Grid{P, Q, r / Q, r % Q});
-  const int off[3] = {0, n, 2 * n};
   for (int r = 0; r < P * Q; ++r) {
     if (phase == 0) build_potrf_plan(plans[r], grids[r], n, NB);
-    else if (phase == 1) build_uinv_plan(plans[r], grids[r], n, NB);
-    else build_ablock_plan(plans[r], grids[r], n, 2 * n + nb_extra, off, NB);
-  }
-  if (phase == 2) {
-    std::vector<int> cnt((size_t)nblk * nblk, 0);
-    for (int r = 0; r < P * Q; ++r) {
-      if (plans[r].host.size() != 4 * plans[r].hblocks.size()) return 20;
-      for (const int4& hb : plans[r].hblocks) {
-        if (owner_of(grids[r], hb.x, hb.y) != r || hb.y > hb.x) return 21;
-        cnt[(size_t)hb.x * nblk + hb.y]++;
-      }
-    }
-    for (int bi = 0; bi < nblk; ++bi)
-      for (int bc = 0; bc <= bi; ++bc)
-        if (cnt[(size_t)bi * nblk + bc] != 1) return 22;
-    return 0;
+    else build_uinv_plan(plans[r], grids[r], n, NB);
   }
   for (int j = 0; j < nblk; ++j) {
     std::vector<int> upd((size_t)nblk * nblk, 0), solved(nblk, 0);
@@ -1240,16 +1337,20 @@ int gpp_dist_potrf(gpp_handle* h, int* info) {
   return GPP_OK;
 }
 
-// Distributed counterpart of gpp_inverse for the elliptic layout: U = L^{-T} (sharded, then replicated) and the
-// sub-blocks of the interior inverse that this rank's Hessian blocks need.  Enables gpp_dist_gn_step.
+// Distributed counterpart of gpp_inverse for the elliptic, Burgers and Eikonal layouts: U = L^{-T} (sharded, then
+// replicated) and the sub-blocks of the interior inverse that this rank's Hessian blocks need for the PDE of that layout.
+// Enables gpp_dist_gn_step for that PDE.
 int gpp_dist_inverse(gpp_handle* h) {
   if (h) cudaSetDevice(h->device);
   if (!h || !h->dist) return -1;
   DistState* d = ds(h);
   GramSlot& s = h->slot[0];
   if (!s.factored) { h->err = "gpp_dist_potrf first"; return -2; }
-  if (s.layout_id != LAY_ELLIPTIC) { h->err = "the sharded GN path supports the elliptic layout only"; return -3; }
+  const int pde = sharded_pde_of_layout(s.layout_id);
+  if (pde < 0) { h->err = "the sharded GN path supports the elliptic, Burgers and Eikonal layouts only"; return -3; }
   CUDA_TRY(h, cudaSetDevice(h->device));
+  d->inverse_ready = false;
+  d->inv_pde = pde;
   int rc = dev_reserve(h, &d->U, (size_t)s.M * s.ld);
   if (rc) return rc;
   rc = make_tensor_map(h, &d->mapU, d->U, s.M, s.M, s.ld);
@@ -1275,13 +1376,19 @@ int gpp_dist_inverse(gpp_handle* h) {
 }
 
 // one iteration of GN_method's loop body (src/PDEs.py:117-120) with the sharded Hessian assembly and the distributed
-// Cholesky of H; every rank ends with the same z and returns the same loss
+// Cholesky of H; every rank ends with the same z and returns the same loss.  The PDE set up by gpp_gn_setup must be the
+// one of the layout gpp_dist_inverse planned for.
 int gpp_dist_gn_step(gpp_handle* h, double step, double* loss) {
   if (h) cudaSetDevice(h->device);
   if (!h || !h->dist) return -1;
   if (!h->gn.ready) { h->err = "gpp_gn_setup first"; return -1; }
-  if (h->gn.pde != PDE_ELLIPTIC) { h->err = "the sharded GN path supports Nonlinear_elliptic only"; return -2; }
+  const int pde = h->gn.pde;
+  if (pde != PDE_ELLIPTIC && pde != PDE_BURGERS && pde != PDE_EIKONAL) {
+    h->err = "the sharded GN path supports Nonlinear_elliptic, Burgers and Eikonal only";
+    return -2;
+  }
   if (!ds(h)->inverse_ready || !h->dist_gn) { h->err = "gpp_dist_inverse first"; return -3; }
+  if (pde != ds(h)->inv_pde) { h->err = "gpp_dist_inverse was built for the Gram layout of another PDE"; return -5; }
   if (!loss) return -4;
   CUDA_TRY(h, cudaSetDevice(h->device));
   return gn_step(h, step, loss);

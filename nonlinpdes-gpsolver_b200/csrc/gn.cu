@@ -183,14 +183,6 @@ sumsq_kernel(const double* __restrict__ a, int na, const double* __restrict__ b,
   if (threadIdx.x == 0) out[0] = sh[0];
 }
 
-struct TermTable {
-  int nz, nslots;
-  int nterms[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS];
-  unsigned char ts[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS][8];
-  unsigned char tp[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS][8];
-  unsigned char tpp[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS][8];
-};
-
 struct HParams {
   TermTable tt;
   int N;
@@ -226,35 +218,38 @@ hess_kernel(const __grid_constant__ HParams a) {
   }
 }
 
-// multi-GPU (elliptic): one launch covers the Hessian blocks (bi, bc) this rank owns.  A sub-blocks of block e sit at rows
-// (4 e + 2 p + p') * nbh of a compact store with leading dimension nbh.  Same term order as hess_kernel:
+// multi-GPU: one launch covers the Hessian blocks (bi, bc) this rank owns.  Row bi * nbh + r of H is (q, i), column
+// bc * nbh + c is (q', j); term t of the pair (q, q') sits at row (4 e + t) * nbh + r of the compact sub-block store
+// (leading dimension nbh).  Same terms in the same order as hess_kernel, e.g. elliptic:
 // H_ij = 2 ((c_i A00) c_j + (c_i A01) 1 + (1 A10) c_j + (1 A11) 1)                       src/PDEs.py:94-102
 __global__ void __launch_bounds__(256)
-hess_blocks_kernel(const int4* __restrict__ blocks, const double* __restrict__ Asub, int nbh, int N,
-                   const double* __restrict__ c0, const double* __restrict__ c1, double* __restrict__ H, long ldH) {
+hess_blocks_kernel(const __grid_constant__ TermTable tt, const int4* __restrict__ blocks, const double* __restrict__ Asub,
+                   int nbh, int N, const double* __restrict__ coef, double* __restrict__ H, long ldH) {
   const int4 b = blocks[blockIdx.z];
-  const int j = blockIdx.x * 64 + (threadIdx.x & 63);
-  const int ibase = blockIdx.y * 16 + (threadIdx.x >> 6) * 4;
-  const int gj = b.y * nbh + j;
-  if (j >= nbh || gj >= N) return;
-  const double* A00 = Asub + (long)(b.z * 4 + 0) * nbh * nbh;
-  const double* A01 = Asub + (long)(b.z * 4 + 1) * nbh * nbh;
-  const double* A10 = Asub + (long)(b.z * 4 + 2) * nbh * nbh;
-  const double* A11 = Asub + (long)(b.z * 4 + 3) * nbh * nbh;
-  const double cj0 = c0[gj], cj1 = c1[gj];
+  const int n = tt.nz * N;
+  const int c = blockIdx.x * 64 + (threadIdx.x & 63);
+  const int rbase = blockIdx.y * 16 + (threadIdx.x >> 6) * 4;
+  const int gc = b.y * nbh + c;
+  if (c >= nbh || gc >= n) return;
+  const int qq = gc / N, j = gc - qq * N;
+  const long sub = (long)nbh * nbh;
 #pragma unroll
   for (int ii = 0; ii < 4; ++ii) {
-    const int i = ibase + ii;
-    const int gi = b.x * nbh + i;
-    if (i >= nbh || gi >= N) break;
-    const double ci0 = c0[gi], ci1 = c1[gi];
-    const long e = (long)i * nbh + j;
+    const int r = rbase + ii;
+    const int gr = b.x * nbh + r;
+    if (r >= nbh || gr >= n) break;
+    const int q = gr / N, i = gr - q * N;
+    const int pr = q * tt.nz + qq;
+    const int nt = tt.nterms[pr];
+    const double* A = Asub + (long)b.z * 4 * sub + (long)r * nbh + c;
     double acc = 0.0;
-    acc += (ci0 * A00[e]) * cj0;
-    acc += (ci0 * A01[e]) * cj1;
-    acc += (ci1 * A10[e]) * cj0;
-    acc += (ci1 * A11[e]) * cj1;
-    H[(long)gi * ldH + gj] = 2.0 * acc;
+    for (int t = 0; t < nt; ++t) {
+      const int s = tt.ts[pr][t], p = tt.tp[pr][t], pp = tt.tpp[pr][t];
+      const double ci = coef[((long)((s * GPP_MAX_BLOCKS + p) * GPP_MAX_ZBLOCKS + q)) * N + i];
+      const double cj = coef[((long)((s * GPP_MAX_BLOCKS + pp) * GPP_MAX_ZBLOCKS + qq)) * N + j];
+      acc += (ci * A[t * sub]) * cj;
+    }
+    H[(long)gr * ldH + gc] = 2.0 * acc;
   }
 }
 
@@ -302,10 +297,10 @@ __global__ void axpy_kernel(double* __restrict__ z, const double* __restrict__ d
   if (i < n) z[i] = z[i] - step * d[i];
 }
 
-void set_kind(GnState& g) {
-  memset(g.coef_kind, 0, sizeof(g.coef_kind));
-  auto K = [&](int s, int p, int q) { g.coef_kind[s][p][q] = 1; };
-  switch (g.pde) {
+void kind_table(int pde, unsigned char (&kind)[GPP_MAX_SLOTS][GPP_MAX_BLOCKS][GPP_MAX_ZBLOCKS]) {
+  memset(kind, 0, sizeof(kind));
+  auto K = [&](int s, int p, int q) { kind[s][p][q] = 1; };
+  switch (pde) {
     case PDE_ELLIPTIC: K(0, 0, 0); K(0, 1, 0); break;
     case PDE_ELLIPTIC_RELAXED: K(0, 0, 0); K(0, 1, 1); break;
     case PDE_BURGERS: K(0, 0, 0); K(0, 0, 1); K(0, 0, 2); K(0, 1, 1); K(0, 2, 2); K(0, 3, 0); break;
@@ -317,9 +312,38 @@ void set_kind(GnState& g) {
   }
 }
 
+void set_kind(GnState& g) { kind_table(g.pde, g.coef_kind); }
+
 int nslots_of(const GnState& g) { return g.pde == PDE_DARCY ? 2 : 1; }
 
 }  // namespace
+
+int pde_nz(int pde) { return (pde == PDE_ELLIPTIC) ? 1 : (pde == PDE_DARCY ? 6 : (pde == PDE_ELLIPTIC_RELAXED ? 2 : 3)); }
+
+// every coefficient kind of a slot lies inside that slot's layout, so the term lists need no layout
+int make_term_table(int pde, TermTable* tt) {
+  if (pde < PDE_ELLIPTIC || pde > PDE_ELLIPTIC_RELAXED) return -1;
+  unsigned char kind[GPP_MAX_SLOTS][GPP_MAX_BLOCKS][GPP_MAX_ZBLOCKS];
+  kind_table(pde, kind);
+  memset(tt, 0, sizeof(*tt));
+  tt->nz = pde_nz(pde);
+  tt->nslots = pde == PDE_DARCY ? 2 : 1;
+  for (int q = 0; q < tt->nz; ++q)
+    for (int qq = 0; qq < tt->nz; ++qq) {
+      const int pr = q * tt->nz + qq;
+      int nt = 0;
+      for (int s = 0; s < tt->nslots; ++s)
+        for (int p = 0; p < GPP_MAX_BLOCKS; ++p)
+          for (int pp = 0; pp < GPP_MAX_BLOCKS; ++pp)
+            if (kind[s][p][q] && kind[s][pp][qq]) {
+              if (nt >= 8) return -1;
+              tt->ts[pr][nt] = s; tt->tp[pr][nt] = p; tt->tpp[pr][nt] = pp;
+              ++nt;
+            }
+      tt->nterms[pr] = nt;
+    }
+  return 0;
+}
 
 int gn_eval_F(gpp_handle* h, const double* d_z, bool with_coef) {
   GnState& g = h->gn;
@@ -372,15 +396,17 @@ int gn_loss(gpp_handle* h, const double* d_z, double* loss_host) {
 
 int gn_hess_blocks(gpp_handle* h, const int4* d_blocks, int nblocks, const double* Asub, int nbh) {
   GnState& g = h->gn;
-  if (g.pde != PDE_ELLIPTIC) { h->err = "sharded Hessian assembly: elliptic only"; return -1; }
+  if (g.pde != PDE_ELLIPTIC && g.pde != PDE_BURGERS && g.pde != PDE_EIKONAL) {
+    h->err = "sharded Hessian assembly: elliptic, Burgers and Eikonal only";
+    return -1;
+  }
+  TermTable tt;
+  if (make_term_table(g.pde, &tt)) { h->err = "term table"; return -1; }
   if (nblocks <= 0) return GPP_OK;
-  const int N = h->N;
-  const double* c0 = g.coef + ((long)((0 * GPP_MAX_BLOCKS + 0) * GPP_MAX_ZBLOCKS + 0)) * N;
-  const double* c1 = g.coef + ((long)((0 * GPP_MAX_BLOCKS + 1) * GPP_MAX_ZBLOCKS + 0)) * N;
   for (int b0 = 0; b0 < nblocks; b0 += 32768) {
     const int nb = (nblocks - b0 < 32768) ? (nblocks - b0) : 32768;
     dim3 grid((nbh + 63) / 64, (nbh + 15) / 16, nb);
-    hess_blocks_kernel<<<grid, 256, 0, h->cur>>>(d_blocks + b0, Asub, nbh, N, c0, c1, g.H, g.ldH);
+    hess_blocks_kernel<<<grid, 256, 0, h->cur>>>(tt, d_blocks + b0, Asub, nbh, h->N, g.coef, g.H, g.ldH);
     h->launches++;
   }
   CUDA_TRY(h, cudaGetLastError());
@@ -444,20 +470,7 @@ int gn_grad_hess(gpp_handle* h) {
   // Hessian
   {
     HParams a{};
-    a.tt.nz = g.nz; a.tt.nslots = ns;
-    for (int q = 0; q < g.nz; ++q)
-      for (int qq = 0; qq < g.nz; ++qq) {
-        int nt = 0;
-        for (int s = 0; s < ns; ++s)
-          for (int p = 0; p < h->slot[s].lay.nblk; ++p)
-            for (int pp = 0; pp < h->slot[s].lay.nblk; ++pp)
-              if (g.coef_kind[s][p][q] && g.coef_kind[s][pp][qq]) {
-                if (nt >= 8) { h->err = "term table overflow"; return -1; }
-                a.tt.ts[q * g.nz + qq][nt] = s; a.tt.tp[q * g.nz + qq][nt] = p; a.tt.tpp[q * g.nz + qq][nt] = pp;
-                ++nt;
-              }
-        a.tt.nterms[q * g.nz + qq] = nt;
-      }
+    if (make_term_table(g.pde, &a.tt)) { h->err = "term table overflow"; return -1; }
     a.N = N; a.coef = g.coef;
     for (int s = 0; s < ns; ++s) { a.A[s] = h->slot[s].Ainv; a.ldA[s] = h->slot[s].ldA; }
     a.H = g.H; a.ldH = g.ldH;

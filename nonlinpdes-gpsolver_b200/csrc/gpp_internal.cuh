@@ -274,8 +274,20 @@ int gn_loss(gpp_handle* h, const double* d_z, double* loss_host);
 int gn_step(gpp_handle* h, double step, double* loss_host);
 int gn_grad_hess(gpp_handle* h);
 int gn_grad(gpp_handle* h);           // t = L^{-T} s and the gradient
-// multi-GPU (elliptic): H blocks listed in d_blocks (int4: bi, bc, index of the 2 x 2 group of A sub-blocks, unused) from
-// the compact sub-block store Asub (blocks of nbh x nbh, leading dimension nbh, order (p, p') = 00, 01, 10, 11)
+// Hessian terms: H[(q, i), (q', j)] = 2 sum_t c_{s p q}[i] A_s[(p, i), (p', j)] c_{s p' q'}[j] over the terms t = (s, p, p')
+// of the unknown-block pair (q, q') (index q * nz + q'), in the order the Hessian kernels sum them
+struct TermTable {
+  int nz, nslots;
+  int nterms[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS];
+  unsigned char ts[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS][8];
+  unsigned char tp[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS][8];
+  unsigned char tpp[GPP_MAX_ZBLOCKS * GPP_MAX_ZBLOCKS][8];
+};
+int pde_nz(int pde);                                   // number of unknown blocks of a PDE id
+int make_term_table(int pde, TermTable* tt);           // host only; -1 on an unknown PDE id
+// multi-GPU: H blocks listed in d_blocks (int4: bi, bc, index e of the block's group of four sub-blocks, unused) from the
+// compact sub-block store Asub (nbh x nbh sub-blocks, leading dimension nbh): element (r, c) of block e takes term t of
+// its unknown-block pair from row (4 e + t) * nbh + r, column c.  Elliptic, Burgers and Eikonal (at most four terms a pair).
 int dist_gn_hess_potrf(gpp_handle* h);   // dist.cu
 // single GPU: the right-looking schedule of the sharded path with one rank (task-list updates, look-ahead streams)
 int potrf_right_looking(gpp_handle* h, double* A, long ld, int n, const TMap2* map);
