@@ -98,6 +98,17 @@ int gpp_gn_coef(gpp_handle* h, int slot, int p, int q, double* c_out, int* prese
 int gpp_predict(gpp_handle* h, int slot, const double* X_test, int N_test, const double* w, double* out);
 /* construct_Theta_test  src/Gram_matrice.py:190-289: out is N_test x M row-major */
 int gpp_theta_test(gpp_handle* h, int slot, const double* X_test, int N_test, double* out);
+/* Posterior variance of the GP solution at the test points (new: the reference returns the posterior mean only):
+ *   var_out[t] = kappa(x_t, x_t) - theta(x_t)^T Theta^{-1} theta(x_t),
+ * theta(x_t) = row t of gpp_theta_test (identity functional at x_t, the slot's operators at the collocation points),
+ * Theta = the matrix the slot holds factorised, nugget included; kappa(x, x) = 1 for both kernels.  This is the squared
+ * power function: |u(x) - extend_sol(x)| <= sqrt(var(x)) |u|_RKHS.  Computed as kappa - |L^{-1} theta|^2 by a blocked
+ * triangular solve against the lower triangle of the factor (valid after gpp_potrf, with or without gpp_inverse; it
+ * does not depend on the GN iterate).  Unclamped: near collocation points it is a difference of two numbers close to
+ * kappa and can come out at -O(1e-13); take sqrt(max(var, 0)).  A row's value depends on that row alone (not on
+ * N_test or the other points).  Works on every handle, sharded ones included (all rows computed locally).
+ * < 0 with gpp_last_error set when the slot is not factored. */
+int gpp_predict_var(gpp_handle* h, int slot, const double* X_test, int N_test, double* var_out);
 
 /* Gaussian_kernel / Anisotropic_Gaussian_kernel methods  src/kernels.py:8-179, vectorised over n pairs:
  * out = L_x(op_x) L_y(op_y) kappa(x, y).  Operator ids: 0 identity, 1 d/dx1, 2 d/dx2, 3 d^2/dx2^2, 4 Laplacian
@@ -149,6 +160,10 @@ int gpp_dist_inverse(gpp_handle* h);
  * method and Darcy are refused); the PDE of gpp_gn_setup must be the one of the layout gpp_dist_inverse planned for,
  * otherwise -5 */
 int gpp_dist_gn_step(gpp_handle* h, double step_size, double* loss);
+/* gpp_predict_var of slot 0 after gpp_dist_potrf with the test points split over the ranks: rank r computes rows
+ * [r c, min(N_test, (r + 1) c)), c = ceil(N_test / world), and one sum all-reduce (zeros elsewhere, so exact) leaves the
+ * whole vector, bit-identical to gpp_predict_var on the same factor, on every rank.  All ranks pass the same points. */
+int gpp_dist_predict_var(gpp_handle* h, const double* X_test, int N_test, double* var_out);
 
 #ifdef __cplusplus
 }

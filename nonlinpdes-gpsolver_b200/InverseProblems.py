@@ -148,3 +148,12 @@ class Darcy_flow2d(_GPProblem):
         self.X_test, self.N_test = X_test, X_test.shape[0]
         self.extended_sol_a = eng.predict(1, X_test, eng.solve_vec(1, self.sol_vec_a))
         self.extended_sol_u = eng.predict(0, X_test, eng.solve_vec(0, self.sol_vec_u))
+
+    def extend_sol_var(self, X_test):
+        """Posterior variances at the test points of the two fields extend_sol predicts (see _GPProblem.extend_sol_var):
+        extended_var_u from Theta_u (slot 0), extended_var_a from Theta_a (slot 1, the field of extended_sol_a)."""
+        self._check_factored()
+        eng = self._engine()
+        X_test = onp.ascontiguousarray(X_test, dtype=onp.float64)
+        self.extended_var_u = eng.predict_var(0, X_test)
+        self.extended_var_a = eng.predict_var(1, X_test)

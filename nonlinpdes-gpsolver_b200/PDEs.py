@@ -299,6 +299,21 @@ class _GPProblem(object):
         self.N_test = X_test.shape[0]
         self.extended_sol = eng.predict(0, X_test, temp)
 
+    def _check_factored(self):
+        if getattr(self, '_state', None) not in ('chol', 'solved'):
+            raise RuntimeError("call Gram_Cholesky() first")
+
+    def extend_sol_var(self, X_test):
+        """Posterior variance of u at the test points (no counterpart in the reference):
+        extended_var = kappa(x, x) - theta(x)^T Theta^{-1} theta(x), theta(x) the row of construct_Theta_test, Theta the
+        factored Gram matrix (nugget included).  sqrt(extended_var) bounds |u - extended_sol| / |u|_RKHS pointwise.  It
+        needs only the factor (available after Gram_Cholesky, before or after GN_method).  Unclamped: near collocation
+        points it can be -O(1e-13); use sqrt(max(var, 0)).  A sharded problem splits the test points over the ranks."""
+        self._check_factored()
+        eng = self._engine()
+        X_test = onp.ascontiguousarray(X_test, dtype=onp.float64)
+        self.extended_var = eng.dist_predict_var(X_test) if self._sharded else eng.predict_var(0, X_test)
+
 
 class Nonlinear_elliptic2d(_GPProblem):
     """-Delta u + alpha*u^m = f in a box (src/PDEs.py:18-208)."""

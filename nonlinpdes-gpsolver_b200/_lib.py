@@ -55,6 +55,7 @@ def _sig(lib):
         "gpp_gn_coef": [H, C.c_int, C.c_int, C.c_int, _dp, _ip],
         "gpp_predict": [H, C.c_int, _dp, C.c_int, _dp, _dp],
         "gpp_theta_test": [H, C.c_int, _dp, C.c_int, _dp],
+        "gpp_predict_var": [H, C.c_int, _dp, C.c_int, _dp],
         "gpp_kernel_eval": [H, C.c_int, _dp, C.c_int, C.c_int, _dp, _dp, _dp, _dp, C.c_long, _dp],
         "gpp_dist_unique_id": [C.POINTER(C.c_ubyte)],
         "gpp_dist_init": [H, C.c_int, C.c_int, C.POINTER(C.c_ubyte)],
@@ -71,6 +72,7 @@ def _sig(lib):
         "gpp_dist_potrf": [H, _ip],
         "gpp_dist_inverse": [H],
         "gpp_dist_gn_step": [H, C.c_double, _dp],
+        "gpp_dist_predict_var": [H, _dp, C.c_int, _dp],
     }
     for name, args in sigs.items():
         fn = getattr(lib, name)
@@ -99,6 +101,13 @@ def _f64(a, shape=None):
     if shape is not None and a.shape != tuple(shape):
         raise ValueError(f"expected shape {shape}, got {a.shape}")
     return a
+
+
+def _test_points(X_test):
+    Xt = _f64(X_test)
+    if Xt.ndim != 2 or Xt.shape[1] != 2 or Xt.shape[0] == 0:
+        raise ValueError(f"X_test must be (N_test, 2) with N_test >= 1, got {Xt.shape}")
+    return Xt
 
 
 def _ptr(a):
@@ -312,6 +321,13 @@ class Engine:
         self._ck(self._lib.gpp_theta_test(self._h, slot, _ptr(Xt), Xt.shape[0], _ptr(out)), "gpp_theta_test")
         return out
 
+    def predict_var(self, slot, X_test):
+        """Posterior variance kappa(x, x) - theta(x)^T Theta^{-1} theta(x) at the test points (unclamped)."""
+        Xt = _test_points(X_test)
+        out = np.empty(Xt.shape[0])
+        self._ck(self._lib.gpp_predict_var(self._h, slot, _ptr(Xt), Xt.shape[0], _ptr(out)), "gpp_predict_var")
+        return out
+
     def kernel_eval(self, kernel, kernel_parameter, op_x, op_y, x1, x2, y1, y2):
         arrs = np.broadcast_arrays(*[np.asarray(a, dtype=np.float64) for a in (x1, x2, y1, y2)])
         shape = arrs[0].shape
@@ -376,6 +392,13 @@ class Engine:
         v = C.c_double()
         self._ck(self._lib.gpp_dist_gn_step(self._h, float(step), C.byref(v)), "gpp_dist_gn_step")
         return float(v.value)
+
+    def dist_predict_var(self, X_test):
+        """predict_var of slot 0 with the test points split over the ranks; the same vector on every rank."""
+        Xt = _test_points(X_test)
+        out = np.empty(Xt.shape[0])
+        self._ck(self._lib.gpp_dist_predict_var(self._h, _ptr(Xt), Xt.shape[0], _ptr(out)), "gpp_dist_predict_var")
+        return out
 
 
 def dist_plan_check(n, NB, P, Q=1, phase=0, nb_extra=0):

@@ -19,6 +19,7 @@ SOURCES = [
     ("gn.cu", ["-fmad=false"]),
     ("capi.cu", []),
     ("dist.cu", []),
+    ("predvar.cu", []),
 ]
 ARCH = ["-gencode", "arch=compute_100a,code=sm_100a"]
 COMMON = ["-O3", "-std=c++17", "-lineinfo", "-Xcompiler", "-fPIC"]

@@ -134,6 +134,7 @@ int gpp_destroy(gpp_handle* h) {
   dev_free(g.rhs_f); dev_free(g.bdy_g); dev_free(g.data_u); dev_free(g.z); dev_free(g.coef); dev_free(g.H); dev_free(g.g);
   dev_free(g.scal);
   for (int s = 0; s < GPP_MAX_SLOTS; ++s) { dev_free(g.F[s]); dev_free(g.s[s]); dev_free(g.t[s]); }
+  dev_free(h->var_W); dev_free(h->var_io); dev_free(h->var_aux);
   if (h->work) cudaFree(h->work);
   if (h->d_info) cudaFree(h->d_info);
   if (h->d_trsv_flag) cudaFree(h->d_trsv_flag);
@@ -579,6 +580,24 @@ int gpp_theta_test(gpp_handle* h, int slot, const double* Xtest, int ntest, doub
   rc = gram_theta_test(h, s, d_xt, ntest, d_o, s.M);
   if (rc) return rc;
   CUDA_TRY(h, cudaMemcpyAsync(out, d_o, sizeof(double) * nout, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+  return GPP_OK;
+}
+
+int gpp_predict_var(gpp_handle* h, int slot, const double* Xtest, int ntest, double* var_out) {
+  NvtxRange nvtx_range("gpp:predict_var");
+  if (h) cudaSetDevice(h->device);
+  if (bad_slot(h, slot)) return -2;
+  if (!Xtest || ntest <= 0 || !var_out) return -3;
+  if (!h->slot[slot].factored) { h->err = "potrf first"; return -4; }
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = dev_alloc(h, &h->var_io, (size_t)3 * ntest);
+  if (rc) return rc;
+  double* d_xt = h->var_io; double* d_var = d_xt + 2 * (size_t)ntest;
+  CUDA_TRY(h, cudaMemcpyAsync(d_xt, Xtest, sizeof(double) * 2 * ntest, cudaMemcpyHostToDevice, h->stream));
+  rc = predict_var(h, slot, d_xt, 0, ntest, d_var);
+  if (rc) return rc;
+  CUDA_TRY(h, cudaMemcpyAsync(var_out, d_var, sizeof(double) * ntest, cudaMemcpyDeviceToHost, h->stream));
   CUDA_TRY(h, cudaStreamSynchronize(h->stream));
   return GPP_OK;
 }

@@ -1375,6 +1375,38 @@ int gpp_dist_inverse(gpp_handle* h) {
   return GPP_OK;
 }
 
+// Posterior variance of slot 0 at N_test test points, split over the ranks: L is complete on every rank after
+// gpp_dist_potrf and the test rows are independent given L, so rank r computes the contiguous rows
+// [r c, min(N_test, (r + 1) c)), c = ceil(N_test / world), writes zeros elsewhere, and one sum all-reduce combines the
+// ranks (adding zeros is exact: every rank ends with the same vector).  Virtual mode runs every rank's rows in turn.
+int gpp_dist_predict_var(gpp_handle* h, const double* Xtest, int ntest, double* var_out) {
+  if (h) cudaSetDevice(h->device);
+  if (!h || !h->dist) return -1;
+  DistState* d = ds(h);
+  GramSlot& s = h->slot[0];
+  if (!s.factored) { h->err = "gpp_dist_potrf first"; return -2; }
+  if (!Xtest || ntest <= 0 || !var_out) return -3;
+  CUDA_TRY(h, cudaSetDevice(h->device));
+  int rc = dev_reserve(h, &h->var_io, (size_t)3 * ntest);
+  if (rc) return rc;
+  double* d_xt = h->var_io; double* d_var = d_xt + 2 * (size_t)ntest;
+  CUDA_TRY(h, cudaMemcpyAsync(d_xt, Xtest, sizeof(double) * 2 * ntest, cudaMemcpyHostToDevice, h->stream));
+  CUDA_TRY(h, cudaMemsetAsync(d_var, 0, sizeof(double) * ntest, h->stream));
+  const int nranks = d->nv > 0 ? d->nv : d->world;
+  const long c = ((long)ntest + nranks - 1) / nranks;
+  for (int r = 0; r < nranks; ++r) {
+    if (d->nv == 0 && r != d->rank) continue;
+    const long r0 = r * c, r1 = std::min<long>(ntest, r0 + c);
+    if (r1 <= r0) continue;
+    rc = predict_var(h, 0, d_xt, (int)r0, (int)(r1 - r0), d_var);
+    if (rc) return rc;
+  }
+  if (d->world > 1) NCCL_TRY(h, ncclAllReduce(d_var, d_var, ntest, ncclDouble, ncclSum, d->comm, h->stream));
+  CUDA_TRY(h, cudaMemcpyAsync(var_out, d_var, sizeof(double) * ntest, cudaMemcpyDeviceToHost, h->stream));
+  CUDA_TRY(h, cudaStreamSynchronize(h->stream));
+  return GPP_OK;
+}
+
 // one iteration of GN_method's loop body (src/PDEs.py:117-120) with the sharded Hessian assembly and the distributed
 // Cholesky of H; every rank ends with the same z and returns the same loss.  The PDE set up by gpp_gn_setup must be the
 // one of the layout gpp_dist_inverse planned for.

@@ -136,6 +136,14 @@ struct gpp_handle {
   cudaEvent_t ev[10];               // [0,1] phase timer, [2..7] GN trace, [8,9] outer (bench) timer
   float t_asm = 0, t_potrf = 0, t_inv = 0, t_step = 0;
   long launches = 0;
+  // posterior variance (predvar.cu): work buffer of one chunk of test rows, its tensor map (re-encoded when the buffer
+  // or the shape changes) and the test points / variance vector / kappa(x, x) scratch of the public calls
+  double* var_W = nullptr;
+  TMap2 var_map{};
+  const double* var_map_base = nullptr;
+  long var_map_rows = 0, var_map_cols = 0, var_map_ld = 0;
+  double* var_io = nullptr;
+  double* var_aux = nullptr;
   // distributed (dist.cu)
   void* dist = nullptr;
   bool dist_gn = false;               // GN steps use the sharded Hessian assembly + distributed Cholesky of H
@@ -267,6 +275,10 @@ int gram_slot_prepare(gpp_handle* h, int slot, int layout, int kernel, const dou
 int gram_assemble(gpp_handle* h, GramSlot& s);
 int gram_predict(gpp_handle* h, GramSlot& s, const double* d_xtest, int ntest, const double* d_w, double* d_out);
 int gram_theta_test(gpp_handle* h, GramSlot& s, const double* d_xtest, int ntest, double* d_out, long ldo);
+
+// ---- predvar.cu: posterior variance d_var[t] = kappa(x_t, x_t) - theta(x_t)^T Theta^{-1} theta(x_t) of the factored
+// slot for the test rows t in [row0, row0 + nrows) of d_xtest (N_test x 2); other entries of d_var are not touched
+int predict_var(gpp_handle* h, int slot, const double* d_xtest, int row0, int nrows, double* d_var);
 
 // ---- gn.cu -----------------------------------------------------------------
 int gn_eval_F(gpp_handle* h, const double* d_z, bool with_coef);

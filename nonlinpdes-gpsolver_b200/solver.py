@@ -124,6 +124,22 @@ class solver_GP(object):
         _say(print_option, f'[Testing...] Number of test points: {X_test.shape[0]}')
         self.eqn.extend_sol(X_test)
 
+    @staticmethod
+    def _max_std(var):
+        return onp.sqrt(onp.max(onp.maximum(var, 0.0)))
+
+    def test_var(self, X_test, print_option=True):
+        """Posterior variance at the test points (extend_sol_var): test_var_all, and for Darcy_flow2d test_var_all = the
+        variance of u and test_var_all_a = that of a."""
+        self.eqn.extend_sol_var(X_test)
+        if hasattr(self.eqn, 'extended_var_u'):
+            self.test_var_all, self.test_var_all_a = self.eqn.extended_var_u, self.eqn.extended_var_a
+            _say(print_option, f'[Test variance] Max posterior standard deviation of u {self._max_std(self.test_var_all)}',
+                 f'[Test variance] Max posterior standard deviation of a {self._max_std(self.test_var_all_a)}')
+        else:
+            self.test_var_all = self.eqn.extended_var
+            _say(print_option, f'[Test variance] Max posterior standard deviation {self._max_std(self.test_var_all)}')
+
     def get_test_error(self, truth, print_option=True):
         self.truth = truth
         self.test_err_all, self.test_max_err, self.test_L2_err = self._abs_max_rms(truth, self.eqn.extended_sol, self.eqn.N_test)

@@ -6,7 +6,10 @@ emulated ranks on one GPU.  Prints one JSON line per repetition with the per-pha
 alpha = 1, nu = 0.02, anisotropic kernel (0.3, 0.05), (t, x) in [0, 1] x [-1, 1]; M = 4 N + N_boundary); its JSON line also
 carries the flops of the Theta^-1 sub-block phase (max over ranks and total), counted with the rule of the plan builder.
 --single: the unsharded class path on the same inputs, with the same per-phase times (the one-GPU baseline at sizes too
-large for --check).  --dump-outputs DIR: loss history, solution and predictions of the last repetition as .npy files."""
+large for --check).  --dump-outputs DIR: loss history, solution and predictions of the last repetition as .npy files.
+--var-points K: after the solves, the posterior variance at K random test points (extend_sol_var, the test points split
+over the ranks), one warm-up call and one timed call; one more JSON line with its time (max over ranks) and N_test M^2 / t.
+With --check it also checks that every rank holds the same vector, bit-identical to gpp_predict_var on its own factor."""
 import argparse, json, math, os, sys, time
 sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import numpy as np
@@ -24,6 +27,7 @@ ap.add_argument("--virtual", type=int, default=0)
 ap.add_argument("--check", action="store_true")
 ap.add_argument("--single", action="store_true", help="unsharded class path on one GPU")
 ap.add_argument("--dump-outputs", default=None, metavar="DIR")
+ap.add_argument("--var-points", type=int, default=0, metavar="K")
 a = ap.parse_args()
 if a.nugget is None:
     a.nugget = 1e-5 if a.pde == "burgers" else 1e-10
@@ -166,6 +170,36 @@ if a.dump_outputs and rank == 0:
     os.makedirs(a.dump_outputs, exist_ok=True)
     for name, v in (("loss_hist", prob.loss_hist), ("sol", prob.sol), ("pred", prob.extended_sol)):
         np.save(os.path.join(a.dump_outputs, name + ".npy"), np.asarray(v, dtype=np.float64))
+
+if a.var_points:
+    Xv = np.random.RandomState(2).uniform(dom[:, 0], dom[:, 1], (a.var_points, 2))
+    for rep in range(2):                                # warm-up, then the timed call
+        if dist is not None:
+            dist.barrier()
+        eng.sync()
+        t0 = time.perf_counter()
+        prob.extend_sol_var(Xv)
+        var_ms = (time.perf_counter() - t0) * 1e3
+    var = prob.extended_var
+    var_fail = 0.0
+    if a.check:
+        same = True
+        if dist is not None:
+            import torch
+            mine = torch.tensor(var, dtype=torch.float64, device="cuda")
+            root = mine.clone()
+            dist.broadcast(root, 0)
+            same = bool(torch.equal(mine, root))
+        var_fail = 0.0 if same and np.array_equal(var, eng.predict_var(0, Xv)) else 1.0
+    var_ms, var_fail = maxred([var_ms, var_fail])
+    if rank == 0:
+        rec = dict(var_points=a.var_points, world=1 if a.single else (a.virtual or world), virtual=bool(a.virtual), N=N, M=M,
+                   NB=a.NB, var_ms=round(var_ms, 2), var_TF=round(a.var_points * M * M / var_ms / 1e9, 2),
+                   var_min=float(var.min()), var_max=float(var.max()))
+        if a.check:
+            rec["var_same_on_ranks_and_single_rank"] = var_fail == 0.0
+        print(json.dumps(rec), flush=True)
+    assert var_fail == 0.0
 
 if a.check:
     L = eng.gram_download(0, 1)                        # every rank holds the whole factor
